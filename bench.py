@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the fake-quantization hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--sweep] [--train]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--sweep] [--train] [--dump-outputs DIR]
 
 A *step* is one pass of the fused uniform fake-quant forward+backward kernel
 (qd_uniform_fwd_bwd, 'complicated' min/max backward) over one 64 Mi-float32
@@ -21,6 +21,12 @@ DESIGN.md "Multi-GPU"), timing is the max over ranks.
 
 --impl reference times the reference's CPU implementation of the path
 (the op-chain port) on the host, same metric and unit.
+
+--dump-outputs DIR writes what the last timed step returned to a caller, q and
+the input gradient, as DIR/q.npy and DIR/grad_input.npy (float32).  Both are
+the same fixed sample of DUMP_ROWS whole buckets (seeded, sorted bucket
+indices), shape (DUMP_ROWS, BUCKET): 32 MB in all.  Inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -40,6 +46,7 @@ LEVELS = 16
 BUCKET = 256
 BYTES_PER_ELEM = 16        # x, g read; q, gout written
 MODE_NAME = "minmax"
+DUMP_ROWS = 1 << 14        # buckets sampled by --dump-outputs: 4 Mi elements per array
 
 
 def load_peaks():
@@ -492,6 +499,17 @@ def cpu_model_quant_ms(sizes, levels, bucket, repeats=3):
     return best * 1e3
 
 
+def dump_outputs(out_dir, q, gout):
+    """The same seeded sample of DUMP_ROWS buckets of q and of the input gradient, as float32 .npy files."""
+    import numpy as np
+    import torch
+    rows = np.sort(np.random.default_rng(0).choice(N_ELEMS // BUCKET, DUMP_ROWS, replace=False))
+    sel = torch.from_numpy(rows).to(q.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("q", q), ("grad_input", gout)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.view(-1, BUCKET).index_select(0, sel).cpu().numpy())
+
+
 # ----------------------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -508,7 +526,11 @@ def main():
     ap.add_argument("--train-steps", type=int, default=40)
     ap.add_argument("--ref-elements", type=int, default=0,
                     help="TEST HOOK for --impl reference: run the CPU arm on fewer elements (the line says so; not a bench value)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the last timed step's outputs to DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -580,6 +602,8 @@ def main():
     ms_per_step = ms / steps
     per_gpu_gbs = N_ELEMS * BYTES_PER_ELEM / (ms_per_step * 1e-3) / 1e9
     value = per_gpu_gbs * world
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, q, gout)
 
     # ---- e2e: host buffers through the C ABI (H2D + kernel + D2H inside the timed region)
     # the pinned buffers are allocated and first touched on the CPUs of this GPU's NUMA node, so that N ranks

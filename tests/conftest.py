@@ -6,6 +6,7 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 
 
 def pytest_configure(config):
@@ -30,9 +31,9 @@ def built_extension():
 
 @pytest.fixture(scope="session")
 def golden():
-    import numpy as np
+    import golden_store
     path = os.path.join(ROOT, "tests", "golden", "reference_vectors.npz")
-    data = np.load(path)
+    data = golden_store.load(path)
     cases = {}
     for row in data["meta"]:
         family, key, kind, n, b, s = str(row).split("|")
@@ -44,9 +45,9 @@ def golden():
 def golden_options():
     """Reference outputs for the options only the NMT loop passes (subtract_mean, max_element, stochastic
     rounding with the reference's own draws): tests/golden/make_golden_options.py."""
-    import numpy as np
+    import golden_store
     path = os.path.join(ROOT, "tests", "golden", "reference_vectors_options.npz")
-    data = np.load(path)
+    data = golden_store.load(path)
     cases = {}
     for row in data["meta"]:
         family, key, kind, n, b, s, sub, mx = str(row).split("|")

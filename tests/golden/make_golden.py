@@ -34,28 +34,10 @@ warnings.filterwarnings("ignore")
 import quantization as Q  # noqa: E402
 import quantization.help_functions as QH  # noqa: E402
 
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from golden_store import make_input, save  # noqa: E402
+
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_vectors.npz")
-
-
-def make_input(kind, n, seed):
-    g = torch.Generator().manual_seed(seed)
-    if kind == "weights":
-        return torch.randn(n, generator=g) * 0.05
-    if kind == "uniform":
-        return torch.rand(n, generator=g) * 2 - 1
-    if kind == "constant":
-        return torch.full((n,), 0.125)
-    if kind == "ties":
-        # bucket-wise values that land x_hat*S exactly on .5 for S=15 and S=3:
-        # x in {0, 1/30, 3/30, ..., 1} scaled so min=0, max=1 inside each bucket.
-        base = torch.tensor([0.0, 1.0] + [(2 * k + 1) / 30.0 for k in range(15)] + [(2 * k + 1) / 6.0 for k in range(3)])
-        reps = (n + base.numel() - 1) // base.numel()
-        return base.repeat(reps)[:n].clone()
-    if kind == "mixed_scale":
-        x = torch.randn(n, generator=g)
-        scale = torch.logspace(-6, 3, n)
-        return x * scale
-    raise ValueError(kind)
 
 
 def uniform_cases():
@@ -81,6 +63,7 @@ def main():
         def __setitem__(self, k, v):            # .numpy() aliases torch storage: snapshot now
             super().__setitem__(k, np.array(v, copy=True))
     store = _CopyStore()
+    recipes = {}                                 # seeded inputs: redrawn at load time (golden_store.py)
     meta = []
 
     # ---------------- uniform forward + scaling state -----------------------
@@ -89,6 +72,7 @@ def main():
         q, sf = Q.uniformQuantization(x, s, bucket_size=b)
         key = f"u{ci}"
         store[key + "_x"] = x.numpy()
+        recipes[key + "_x"] = ("input", kind, n, 1000 + ci)
         store[key + "_q"] = q.numpy()
         store[key + "_alpha"] = sf.alpha.reshape(-1).numpy()
         store[key + "_beta"] = sf.beta.reshape(-1).numpy()
@@ -106,6 +90,7 @@ def main():
         # inverse scaling of an arbitrary row tensor
         y = torch.rand(xh.size(), generator=torch.Generator().manual_seed(7 + ci))
         store[key + "_inv_in"] = y.reshape(-1).numpy()
+        recipes[key + "_inv_in"] = ("rand", "-", y.numel(), 7 + ci)
         store[key + "_inv_out"] = sf2.inv_scale_down(y).reshape(-1).numpy()
         meta.append(("uniform", key, kind, n, -1 if b is None else b, s))
 
@@ -133,6 +118,7 @@ def main():
         key = f"c{ci}"
         store[key + "_x"] = x.numpy()
         store[key + "_g"] = g.numpy()
+        recipes[key + "_x"], recipes[key + "_g"] = ("input", "weights", n, 2000 + ci), ("randn", "-", n, 3000 + ci)
         store[key + "_gout"] = (g + cap["r"].view(-1)).numpy()
         meta.append(("minmax_bwd", key, "weights", n, b, s))
 
@@ -156,6 +142,7 @@ def main():
             pts = torch.tensor([0.0, 0.2, 0.6, 1.0])   # x_hat hits exact midpoints / equidistant cases
         key = f"n{ci}"
         store[key + "_x"] = x.numpy()
+        recipes[key + "_x"] = ("input", kind, n, 4000 + ci)
         store[key + "_points"] = pts.numpy()
         # direct path = nearest rule
         q, idx, sfn = Q.nonUniformQuantization(x, pts, bucket_size=b)
@@ -177,6 +164,7 @@ def main():
         Q.USE_CUDA = False
         gi, gp = f.backward(g)
         store[key + "_g"] = g.numpy()
+        recipes[key + "_g"] = ("randn", "-", n, 5000 + ci)
         store[key + "_gpoints2"] = gp.numpy()
         meta.append(("nonuniform", key, kind, n, -1 if b is None else b, K))
 
@@ -187,6 +175,7 @@ def main():
         pts = QH.initialize_quantization_points(x, sf, K)
         key = f"p{ci}"
         store[key + "_x"] = x.numpy()
+        recipes[key + "_x"] = ("input", "weights", n, 6000 + ci)
         store[key + "_points"] = pts.numpy()
         meta.append(("init_points", key, "weights", n, -1 if b is None else b, K))
 
@@ -198,12 +187,11 @@ def main():
         key = f"h{ci}"
         for j, p in enumerate(params):
             store[f"{key}_x{j}"] = p.numpy()
+            recipes[f"{key}_x{j}"] = ("input", "weights", p.numel(), 7000 + 10 * ci + j)
         store[key + "_mean_bits"] = np.array([mbl], dtype=np.float64)
         meta.append(("huffman", key, "weights", len(params), -1 if b is None else b, s))
 
-    store = {k: np.array(v, copy=True) for k, v in store.items()}
-    store["meta"] = np.array(["|".join(str(v) for v in m) for m in meta])
-    np.savez_compressed(OUT, **store)
+    save(OUT, store, recipes, meta)
     print("wrote", OUT, os.path.getsize(OUT) // 1024, "KiB;", len(meta), "cases; torch", torch.__version__,
           "numpy", np.__version__)
 

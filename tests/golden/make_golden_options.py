@@ -29,7 +29,7 @@ warnings.filterwarnings("ignore")
 import quantization as Q  # noqa: E402
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-from make_golden import make_input  # noqa: E402  (same seeded input families)
+from golden_store import make_input, save  # noqa: E402  (same seeded input families)
 
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_vectors_options.npz")
 
@@ -48,7 +48,7 @@ def expected_size(n, b):
 
 
 def main():
-    store, meta = {}, []
+    store, recipes, meta = {}, {}, []       # recipes: seeded inputs, redrawn at load time (golden_store.py)
 
     def put(k, v):
         store[k] = np.array(v, copy=True)
@@ -66,6 +66,7 @@ def main():
                         q, sf = Q.uniformQuantization(x, s, bucket_size=b, subtract_mean=sub, max_element=mx)
                         key = f"o{ci}"
                         put(key + "_x", x.numpy())
+                        recipes[key + "_x"] = ("input", kind, n, 8000 + ci)
                         put(key + "_q", q.numpy())
                         put(key + "_alpha", sf.alpha.reshape(-1).numpy())
                         put(key + "_beta", sf.beta.reshape(-1).numpy())
@@ -78,6 +79,7 @@ def main():
                         if s == 16:                                  # inverse scaling (with the mean added back, :148)
                             y = torch.rand(xh.size(), generator=torch.Generator().manual_seed(11 + ci))
                             put(key + "_inv_in", y.reshape(-1).numpy())
+                            recipes[key + "_inv_in"] = ("rand", "-", y.numel(), 11 + ci)
                             put(key + "_inv_out", sf2.inv_scale_down(y).reshape(-1).numpy())
                         meta.append(("pre_uniform", key, kind, n, -1 if b is None else b, s, int(sub), repr(float(mx)) if mx is not False else "no"))
                         ci += 1
@@ -94,6 +96,7 @@ def main():
                         q, idx, sf = Q.nonUniformQuantization(x, pts, bucket_size=b, subtract_mean=sub, max_element=mx)
                         key = f"v{ci}"
                         put(key + "_x", x.numpy())
+                        recipes[key + "_x"] = ("input", kind, n, 9000 + ci)
                         put(key + "_points", pts.numpy())
                         put(key + "_q", q.numpy())
                         put(key + "_idx", idx.numpy())
@@ -118,13 +121,13 @@ def main():
                         key = f"r{ci}"
                         put(key + "_x", x.numpy())
                         put(key + "_u", u.reshape(-1).numpy())
+                        recipes[key + "_x"], recipes[key + "_u"] = ("input", kind, n, 10000 + ci), ("rand", "-", u.numel(), 77000 + ci)
                         put(key + "_q", q.numpy())
                         put(key + "_mean", np.array([float(sf.mean_tensor)], dtype=np.float32))
                         meta.append(("stochastic", key, kind, n, -1 if b is None else b, s, int(sub), repr(float(mx)) if mx is not False else "no"))
                         ci += 1
 
-    store["meta"] = np.array(["|".join(str(v) for v in m) for m in meta])
-    np.savez_compressed(OUT, **store)
+    save(OUT, store, recipes, meta)
     print("wrote", OUT, os.path.getsize(OUT) // 1024, "KiB;", len(meta), "cases; torch", torch.__version__, "numpy", np.__version__)
 
 

@@ -148,6 +148,20 @@ def _free_port():
     return port
 
 
+def _spawn_host_ranks(fn, args, world):
+    """Starts the ranks with CUDA_VISIBLE_DEVICES empty, so that they are host processes on any machine (with one GPU,
+    rank 1 would otherwise ask for cuda:1).  It is set before they start: importing the package already queries CUDA."""
+    saved = os.environ.get("CUDA_VISIBLE_DEVICES")
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""
+    try:
+        mp.spawn(fn, args=args, nprocs=world, join=True)
+    finally:
+        if saved is None:
+            del os.environ["CUDA_VISIBLE_DEVICES"]
+        else:
+            os.environ["CUDA_VISIBLE_DEVICES"] = saved
+
+
 def _ddp_worker(rank, world, port, ret):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
     from quantized_distillation_b200 import distributed as D
@@ -174,7 +188,7 @@ def test_ddp_replicas_stay_identical_gloo_world2():
     port = _free_port()
     with mp.Manager() as mgr:
         ret = mgr.dict()
-        mp.spawn(_ddp_worker, args=(world, port, ret), nprocs=world, join=True)
+        _spawn_host_ranks(_ddp_worker, (world, port, ret), world)
         assert ret[0] is True and ret[1] is True
 
 
@@ -233,7 +247,7 @@ def test_flat_data_parallel_gloo_world2_matches_single_process():
     port = _free_port()
     with mp.Manager() as mgr:
         ret = mgr.dict()
-        mp.spawn(_flat_worker, args=(world, port, ret), nprocs=world, join=True)
+        _spawn_host_ranks(_flat_worker, (world, port, ret), world)
         assert ret[0] is True and ret[1] is True
         dp = ret["params"]
     torch.manual_seed(1234)
